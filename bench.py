@@ -34,6 +34,12 @@ sys.path.insert(0, ROOT)
 
 TILE = 1024
 QP = 27
+DUMP_SAMPLES = 1 << 22      # bytes of RGB per dumped array: 16 MB as float32
+
+
+def dump_sample_index(nbytes):
+    """The byte offsets --dump-outputs samples: fixed by the seed and the picture size alone."""
+    return np.sort(np.random.default_rng(0xB200).integers(0, nbytes, min(DUMP_SAMPLES, nbytes)))
 
 
 def log(*a):
@@ -189,7 +195,11 @@ def main():
     ap.add_argument("--no-ctb64", action="store_true", help="skip the additional CTB 64 measurement (x265's default CTB size)")
     ap.add_argument("--ctb", type=int, default=5, choices=[4, 5, 6], help="log2 CTB size of the synthetic tiles (5 = the benchmark workload)")
     ap.add_argument("--front-end", default="device", choices=["device", "host"], help="where CABAC runs: GPU (one warp per WPP sub-stream) or host cores")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the RGB of the last timed step of the device leg (rgb.npy) and of the e2e legs "
+                    f"(rgb_e2e.npy) as float32, each a fixed seeded sample of {DUMP_SAMPLES} bytes of the picture, so that two builds can be compared")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     warmup = max(3, args.warmup)
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -293,10 +303,14 @@ def main():
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(stream)
         for _ in range(args.steps):
-            device_step()
+            rgb_dev = device_step()
         e1.record(stream)
         barrier()
         dev_ms = max_over_ranks(e0.elapsed_time(e1)) / args.steps
+        dump_dev = None
+        if args.dump_outputs and rank == 0:
+            flat = rgb_dev.reshape(-1)
+            dump_dev = flat[torch.from_numpy(dump_sample_index(flat.numel())).to(dev)].float().cpu().numpy()
         # ---- leg B: end to end through the C ABI, host buffers in, page-locked host RGB out (wall clock around a synchronised region)
         barrier()
         t0 = time.perf_counter()
@@ -387,10 +401,14 @@ def main():
     }
     # ---- parity inside the bench + CPU baseline: the unmodified reference decodes the top-left sub-grid of the SAME tiles
     line["rgb_md5"] = hashlib.md5(host_out.tobytes()).hexdigest()    # full 16384x16384 RGB; the reference arm prints the md5 of its own result
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "rgb.npy"), dump_dev)
+        np.save(os.path.join(args.dump_outputs, "rgb_e2e.npy"), host_out.reshape(-1)[dump_sample_index(host_out.size)].astype(np.float32))
     if not args.no_cpu_baseline:
         sub = min(side, args.ref_sample_side)
         dump = f"/dev/shm/b200_bench_ref_{os.getpid()}.rgb"
-        res, why = reference_arm(side, sub, 2, 1, cores, dump=dump, log2_ctb=args.ctb)
+        res, why = reference_arm(side, sub, args.steps, 1, cores, dump=dump, log2_ctb=args.ctb)
         if res:
             ref = np.fromfile(dump, dtype=np.uint8).reshape(sub * TILE, sub * TILE * 3)
             os.unlink(dump)
@@ -409,7 +427,7 @@ def main():
     if world == 1 and not args.no_plugin_leg and args.front_end == "device":
         for key, extra in (("e2e_plugin", []), ("e2e_plugin_n2", ["--lib", "libheif_ref_b200.so"])):
             dump = f"/dev/shm/b200_bench_plug_{os.getpid()}.rgb"
-            res, why = reference_arm(side, side, 3, 2, side * side, dump=dump, log2_ctb=args.ctb, extra=["--decoder", "b200"] + extra)
+            res, why = reference_arm(side, side, args.steps, 2, side * side, dump=dump, log2_ctb=args.ctb, extra=["--decoder", "b200"] + extra)
             if res:
                 got = np.fromfile(dump, dtype=np.uint8)
                 os.unlink(dump)
@@ -423,12 +441,12 @@ def main():
             t64 = make_tiles(my_idx, workers=max(4, cores), log2_ctb=6)
             dec.decode_grid_to_rgb_host(t64, side, nrows, lb.CHROMA_INTERLEAVED_RGB, out=my_out)
             ts = []
-            for _ in range(3):
+            for _ in range(args.steps):
                 t0 = time.perf_counter(); dec.decode_grid_to_rgb_host(t64, side, nrows, lb.CHROMA_INTERLEAVED_RGB, out=my_out); ts.append(time.perf_counter() - t0)
             s64 = dec.stats()
             line["ctb64"] = {"e2e_mp_s": pixels / 1e6 / (sum(ts) / len(ts)), "e2e_ms_per_step": 1e3 * sum(ts) / len(ts), "entropy_ms": s64.entropy_ms, "recon_ms": s64.recon_ms,
                              "deblock_ms": s64.deblock_ms, "sao_paste_ms": s64.sao_ms, "bits_per_pixel": 8.0 * s64.bitstream_bytes / my_px,
-                             "note": "same pictures, same QP, coded with CTB 64 (x265 default); 3 e2e steps after 1 warm-up"}
+                             "note": f"same pictures, same QP, coded with CTB 64 (x265 default); {args.steps} e2e steps after 1 warm-up"}
         except Exception as e:  # noqa: BLE001
             line["ctb64"] = {"error": str(e)[:200]}
     print(json.dumps(line))

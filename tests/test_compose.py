@@ -1,16 +1,15 @@
 """Overlay compositing (SURVEY 8 a11) and nearest-neighbour scaling (a12).
 
 CPU: the C restatement (oracle/color_oracle.c) against the UNMODIFIED reference (HeifPixelImage::overlay /
-scale_nearest_neighbor, libheif/image/pixelimage.cc:1637-1972) -- needs oracle/_ref built from /root/reference.
+scale_nearest_neighbor, libheif/image/pixelimage.cc:1637-1972), whose results are stored in
+tests/golden/reference_outputs.json (util.reference_fingerprint).
 GPU: the CUDA kernels (libheif_b200/csrc/b200_compose.cu) against the restatement, bit-exact.
 """
 import os
 import numpy as np
 import pytest
 
-from util import ref_plugin
-
-needs_ref = pytest.mark.skipif(ref_plugin() is None, reason="oracle/_ref reference build not present")
+from util import fingerprint, reference_fingerprint
 
 OVERLAY_CASES = [
     # (canvas w, h, background, [(child w, h, alpha?, dx, dy), ...])
@@ -73,27 +72,23 @@ def _out_plane_sizes(cs, chroma, ow, oh, nplanes, alpha):
     return sizes + ([(ow, oh)] if alpha else [])
 
 
-@needs_ref
 @pytest.mark.parametrize("case", range(len(OVERLAY_CASES)))
 def test_overlay_oracle_matches_reference(case):
     from oracle import bindings as ob
     cw, ch, bkg, spec = OVERLAY_CASES[case]
     kids = _children(spec, 100 + case)
-    ref = ob.ref_overlay(cw, ch, bkg, kids)
     got = ob.oracle_overlay(cw, ch, bkg, kids)
-    assert np.array_equal(ref, got)
+    assert fingerprint(got) == reference_fingerprint("ref_overlay", cw, ch, bkg, kids)
 
 
-@needs_ref
 @pytest.mark.parametrize("case", range(len(SCALE_CASES)))
 def test_scale_oracle_matches_reference(case):
     from oracle import bindings as ob
     cs, chroma, bpp, w, h, ow, oh, alpha = SCALE_CASES[case]
     planes, comps = _scale_planes(cs, chroma, bpp, w, h, alpha, 200 + case)
-    ref = ob.ref_scale_nn(cs, chroma, bpp, planes, w, h, ow, oh, alpha)
     sizes = _out_plane_sizes(cs, chroma, ow, oh, len(planes), alpha)
     got = np.concatenate([ob.oracle_scale_plane(p, sw, sh_, (w, h), (ow, oh), c).reshape(-1).view(np.uint8) for p, c, (sw, sh_) in zip(planes, comps, sizes)])
-    assert np.array_equal(ref, got)
+    assert fingerprint(got) == reference_fingerprint("ref_scale_nn", cs, chroma, bpp, planes, w, h, ow, oh, alpha)
 
 
 @pytest.mark.gpu

@@ -7,7 +7,14 @@ import sys
 
 import pytest
 
+from oracle import bindings as ob
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+# md5 of the RGB24 heif_decode_image of the unmodified reference (CPU decoder plugin) returns for the 4 x 4 grid of bench
+# tiles run_bench decodes: `python -m oracle.ref_arm --side 4 --sub 4` prints it as rgb_md5
+REFERENCE_RGB_MD5_4X4 = "1c31ae3b1f537bac349d093950bfc0df"
+# bench.py compares with the reference in the run where the reference build exists
+have_ref = bool(os.path.exists(os.path.join(ob.REF, "libheif_ref.so")) and os.path.exists(os.path.join(ob.REF, "liboracle_plugin.so")) and ob.avcodec_dir())
 
 
 def run_bench(n, port):
@@ -26,17 +33,20 @@ def test_two_gpus_equal_one_gpu_equal_reference(cuda):
         pytest.skip("needs 2 GPUs")
     one = run_bench(1, 29631)
     two = run_bench(2, 29632)
-    assert one["parity_checked"] and two["parity_checked"], (one.get("parity"), two.get("parity"))
-    assert one["rgb_md5"] == two["rgb_md5"]
+    assert one["rgb_md5"] == two["rgb_md5"] == REFERENCE_RGB_MD5_4X4
+    assert one["parity_checked"] == two["parity_checked"] == have_ref, (one.get("parity"), two.get("parity"))
     assert two["n_gpus"] == 2
 
 
 @pytest.mark.gpu
 def test_bench_checks_itself_against_the_reference(cuda):
-    """1 GPU: the bench line carries parity_checked = true (GPU RGB == heif_decode_image of the unmodified reference)."""
+    """1 GPU: the bench's RGB is what heif_decode_image of the unmodified reference returns (stored md5), and where the
+    reference build exists the bench line carries parity_checked = true from its own in-run comparison."""
     one = run_bench(1, 29633)
-    assert one["parity_checked"] is True, one.get("parity")
-    assert one["parity"]["mismatching_bytes"] == 0
+    assert one["rgb_md5"] == REFERENCE_RGB_MD5_4X4
+    if have_ref:
+        assert one["parity_checked"] is True, one.get("parity")
+        assert one["parity"]["mismatching_bytes"] == 0
 
 
 def run_config5(n, port, dump):

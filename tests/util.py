@@ -1,5 +1,8 @@
 """Shared helpers for the test-suite (test infrastructure; may import oracle/)."""
+import atexit
 import ctypes as C
+import hashlib
+import json
 import os
 import sys
 
@@ -11,6 +14,72 @@ if ROOT not in sys.path:
 from oracle import bindings as ob  # noqa: E402
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
+REFERENCE_OUTPUTS = os.path.join(GOLDEN, "reference_outputs.json")
+
+
+def _feed(h, v):
+    if isinstance(v, np.ndarray):
+        h.update(f"a{v.dtype.str}{v.shape};".encode())
+        h.update(np.ascontiguousarray(v).tobytes())
+    elif isinstance(v, (list, tuple)):
+        h.update(b"(")
+        for x in v:
+            _feed(h, x)
+        h.update(b")")
+    else:
+        h.update(f"{v!r};".encode())
+
+
+def fingerprint(*parts):
+    """Digest of dtype, shape and bytes of every array in parts (and of every other value by repr): equal fingerprints
+    mean np.array_equal on every array and equality of everything else."""
+    h = hashlib.sha256()
+    _feed(h, parts)
+    return h.hexdigest()[:32]
+
+
+_stored = None
+
+
+def _write_reference_outputs():
+    with open(REFERENCE_OUTPUTS, "w") as f:
+        json.dump(dict(sorted(_stored.items())), f, indent=0)
+        f.write("\n")
+
+
+def _reference_outputs():
+    global _stored
+    if _stored is None:
+        if os.environ.get("B200_RECORD_REFERENCE"):
+            _stored = {}
+            atexit.register(_write_reference_outputs)
+        else:
+            with open(REFERENCE_OUTPUTS) as f:
+                _stored = json.load(f)
+    return _stored
+
+
+def reference_fingerprint(name, *args, **kw):
+    """fingerprint() of what the unmodified reference libheif returns for oracle.bindings.<name>(*args, **kw): for
+    ref_postprocess the output bytes, width and height; for the others the whole result.
+
+    The fingerprints are stored in tests/golden/reference_outputs.json, keyed by a digest of the call, so the comparison
+    with the reference runs wherever the tests run.  Where the reference build (oracle/_ref) exists, the reference is also
+    run and must agree with what is stored; with B200_RECORD_REFERENCE=1 its results replace the file instead:
+        B200_RECORD_REFERENCE=1 python -m pytest tests/test_color_oracle.py tests/test_compose.py -m "not gpu"
+    """
+    key = fingerprint(name, args, sorted(kw.items()))
+    stored = _reference_outputs()
+    if ob.ref_plugin() is not None:
+        r = getattr(ob, name)(*args, **kw)
+        fp = fingerprint(*(r[:3] if name == "ref_postprocess" else (r,)))
+        if os.environ.get("B200_RECORD_REFERENCE"):
+            stored[key] = fp
+        else:
+            assert stored.get(key) == fp, f"{name}: the reference build disagrees with tests/golden/reference_outputs.json"
+        return fp
+    assert key in stored, f"{name}: no stored reference output for this call (see util.reference_fingerprint)"
+    return stored[key]
 
 
 def lcg_plane(seed, h, w, lo, hi):
